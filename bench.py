@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot-path benchmark (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|...] [--dump-outputs DIR]
 
 One "step" = one CSR SpMM (sum) pass over the synthetic matrix of BASELINE.json configs[1]:
 1M x 1M (per GPU), ~16 nnz/row, dense operand F=128 bf16 (SURVEY §8d generator G2 / G5).
@@ -351,6 +351,8 @@ def run_ours(args, w):
     ev1.record()
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, rank, world)
     if world > 1:
         dist.barrier()
 
@@ -523,6 +525,25 @@ def run_ours(args, w):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 48 << 20   # all ranks together; row indices add 8 bytes a row
+
+
+def dump_outputs(out_dir, out, rank, world):
+    """What the last timed step returned to its caller, as float32 .npy files: a fixed, seeded sample of its rows
+    (`out.npy`) and their indices (`out_rows.npy`, float64); with several ranks, one pair per rank (`out_rank<r>`).
+    The inputs depend on the arguments only, so two builds can be compared file by file."""
+    import numpy as np
+    import torch
+    M, F = out.size(0), out[0].numel()
+    n = min(M, max(1, DUMP_BYTES // (4 * F * world)))
+    rows = torch.randperm(M, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    tag = "out" if world == 1 else f"out_rank{rank}"
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / f"{tag}.npy", out[rows.to(out.device)].float().cpu().numpy())
+    np.save(d / f"{tag}_rows.npy", rows.double().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -751,7 +772,13 @@ def main():
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary north_star targets (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded row sample of the last step's output to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":   # that arm times a row prefix sized by a clock calibration
+        ap.error("--dump-outputs writes what the GPU path computed; it is not available with --impl reference")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

@@ -1,5 +1,6 @@
-"""Build the reference's OWN CPU operators for the hot path from the sources where they lie under
-/root/reference (read-only; nothing is copied into this repo) into oracle/_ref/:
+"""Build the reference's OWN CPU operators for the hot path from a checkout of the reference (rusty1s/pytorch_sparse,
+read-only; nothing is copied into this repo) into oracle/_ref/. The checkout is $TSB200_REFERENCE or, when that is
+unset, the directory `reference` beside this repository:
 
     _spmm_cpu.so      <- csrc/spmm.cpp + csrc/cpu/spmm_cpu.cpp
     _convert_cpu.so   <- csrc/convert.cpp + csrc/cpu/convert_cpu.cpp
@@ -9,8 +10,9 @@ Recipe: g++ directly on those files against the installed libtorch headers (no s
 flags as the reference's setup.py:67-83 (-O3 -fopenmp -DAT_PARALLEL_OPENMP). OpenMP is NOT passed
 at link time (this image's g++ has no libgomp.spec; libtorch already provides libgomp).
 
-oracle/_ref is git-ignored but travels to the GPU box with the snapshot. TEST / BASELINE
-INFRASTRUCTURE ONLY (see oracle/__init__.py).
+oracle/_ref is git-ignored; where no readable checkout exists nothing is built, the reference-suite test skips and
+the other tests rely on the outputs of the reference stored under tests/golden/. TEST / BASELINE INFRASTRUCTURE ONLY
+(see oracle/__init__.py).
 """
 from __future__ import annotations
 
@@ -20,8 +22,9 @@ import sys
 from concurrent.futures import ThreadPoolExecutor
 from pathlib import Path
 
-REF = Path(os.environ.get("TSB200_REFERENCE", "/root/reference"))
-OUT = Path(__file__).resolve().parent / "_ref"
+ROOT = Path(__file__).resolve().parent.parent
+OUT = ROOT / "oracle" / "_ref"
+REF = Path(os.environ.get("TSB200_REFERENCE") or ROOT.parent / "reference")
 
 LIBS = {
     "_spmm_cpu": ["csrc/spmm.cpp", "csrc/cpu/spmm_cpu.cpp"],
@@ -62,8 +65,8 @@ REF_TESTS = ["test_matmul.py", "test_spmm.py", "test_spspmm.py", "test_coalesce.
 
 def stage_tests() -> Path:
     """Stage the reference's own test files for the hot path, byte for byte, next to its compiled operators in
-    oracle/_ref/ref_tests/ (git-ignored: they never enter this repo's history, but travel to the GPU box, where
-    tests/test_reference_suite_gpu.py runs them unmodified against pytorch_sparse_b200)."""
+    oracle/_ref/ref_tests/ (git-ignored: they never enter this repo's history; tests/test_reference_suite_gpu.py runs
+    them unmodified against pytorch_sparse_b200 where they have been staged)."""
     import shutil
     dst = OUT / "ref_tests"
     dst.mkdir(parents=True, exist_ok=True)
@@ -72,9 +75,18 @@ def stage_tests() -> Path:
     return dst
 
 
+def sources_available() -> bool:
+    """True when REF is a readable checkout of the reference (an unreadable one is treated as absent)."""
+    try:
+        return (REF / "csrc/cpu/spmm_cpu.cpp").is_file()
+    except OSError:
+        return False
+
+
 def build() -> Path:
-    if not (REF / "csrc/cpu/spmm_cpu.cpp").exists():
-        raise FileNotFoundError(f"{REF} not present (the GPU box uses the prebuilt oracle/_ref)")
+    if not sources_available():
+        raise FileNotFoundError(f"reference sources not found in {REF} "
+                                "(set TSB200_REFERENCE to a checkout of the reference)")
     OUT.mkdir(parents=True, exist_ok=True)
     with ThreadPoolExecutor(max_workers=3) as ex:
         list(ex.map(_one, LIBS.items()))

@@ -1,22 +1,22 @@
-"""Generate tests/golden/*.pt by running the UNMODIFIED reference (rusty1s/pytorch_sparse @ 91feaa5)
-in this container:
+"""Generate tests/golden/*.pt by running the UNMODIFIED reference (rusty1s/pytorch_sparse @ 91feaa5), from a
+read-only checkout ($TSB200_REFERENCE, else `reference` beside this repository; see oracle/build_ref.py):
 
-  * its 12 CPU operator libraries compiled from /root/reference/csrc (oracle/build_ref.build_full,
-    into /tmp, nothing copied into the repo),
-  * its Python package imported from a scratch copy of /root/reference/torch_sparse (the package
-    loads its .so files from its own directory, torch_sparse/__init__.py:8-21, and /root/reference
-    is read-only),
+  * its 12 CPU operator libraries compiled from its csrc/ (oracle/build_ref.build_full, into a build cache
+    in the system's temporary directory, nothing copied into the repo),
+  * its Python package imported from a scratch copy of its torch_sparse/ (the package loads its .so files
+    from its own directory, torch_sparse/__init__.py:8-21),
   * `torch_scatter` provided by oracle/torch_scatter_standin (third-party, absent, unpinned; only the
     coalesce VALUE reductions and nothing else on the fixtures below go through it),
   * SpSpMM arithmetic by torch.sparse.mm of the installed PyTorch (third-party; torch 2.11.0+cu128).
 
     python oracle/gen_golden.py            # rewrites tests/golden/
 
-The fixtures hold inputs AND the reference's outputs, so the GPU box (where /root/reference does not
-exist) can check both the oracle and the CUDA path against the reference itself.
+The fixtures hold inputs AND the reference's outputs (no file over 1 MB: the larger ones keep a seeded sample of
+rows), so the tests check both the oracle and the CUDA path against the reference itself without it.
 """
 from __future__ import annotations
 
+import atexit
 import shutil
 import sys
 import tempfile
@@ -27,16 +27,19 @@ import torch
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 GOLD = ROOT / "tests" / "golden"
-REF = Path("/root/reference")
-FULL = Path("/tmp/tsb200_ref_full")
 
 
 def import_reference():
     from oracle import build_ref
-    build_ref.build_full(FULL)
+    if not build_ref.sources_available():
+        raise SystemExit(f"no readable checkout of the reference in {build_ref.REF} (set TSB200_REFERENCE)")
+    ref = build_ref.REF
+    full = Path(tempfile.gettempdir()) / "tsb200_ref_full"   # reused: libraries newer than their sources are kept
+    build_ref.build_full(full)
     scratch = Path(tempfile.mkdtemp(prefix="tsb200_refpkg_"))
-    shutil.copytree(REF / "torch_sparse", scratch / "torch_sparse")
-    for so in FULL.glob("*.so"):
+    atexit.register(shutil.rmtree, scratch, ignore_errors=True)
+    shutil.copytree(ref / "torch_sparse", scratch / "torch_sparse")
+    for so in full.glob("*.so"):
         shutil.copy(so, scratch / "torch_sparse" / so.name)
     sys.path.insert(0, str(scratch))
     sys.path.insert(0, str(ROOT / "oracle" / "torch_scatter_standin"))
@@ -115,7 +118,10 @@ def main():
             c[f"min_{tag}"], c[f"argmin_{tag}"] = torch.ops.torch_sparse.spmm_min(rowptr, col, v, mat)
             c[f"max_{tag}"], c[f"argmax_{tag}"] = torch.ops.torch_sparse.spmm_max(rowptr, col, v, mat)
         cases[f"{str(dtype).split('.')[-1]}_K{K}"] = c
-    torch.save({"meta": meta, "cases": cases}, GOLD / "spmm_medium.pt")
+    # stored: the special rows (empty, longer than a segment) and a seeded sample of the others
+    keep = keep_rows(M, (0, 5, 6, 7, 17, 95), 16, seed=9)
+    cases = {k: sample_spmm_rows(c, keep) for k, c in cases.items()}
+    torch.save({"meta": dict(meta, rows=f"{keep.numel()} of {M} rows"), "cases": cases}, GOLD / "spmm_medium.pt")
 
     # ---- (c) storage views: sort-on-construct, rowptr, csr2csc, colptr (storage.py:149-162, 369-429) ----
     g = torch.Generator().manual_seed(21)
@@ -233,6 +239,7 @@ def main():
     gen_next_rows2(ts, meta)
     gen_spspmm2(ts, meta)
     gen_grads(ts, meta)
+    gen_reference_ops(meta)
 
     sizes = {p.name: p.stat().st_size for p in sorted(GOLD.glob("*.pt"))}
     print("wrote", sizes, "total", sum(sizes.values()))
@@ -290,9 +297,75 @@ def gen_spspmm2(ts, meta):
         va = torch.randn(ra.numel(), generator=g).to(dtype)
         vb = torch.randn(rb.numel(), generator=g).to(dtype)
         ic, vc = ts.spspmm(torch.stack([ra, ca]), va, torch.stack([rb, cb]), vb, M, Kd, N)
-        cases[name] = dict(indexA=torch.stack([ra, ca]), valueA=va, indexB=torch.stack([rb, cb]), valueB=vb,
-                           M=M, K=Kd, N=N, indexC=ic, valueC=vc)
-    torch.save({"meta": meta, "cases": cases}, GOLD / "spspmm2.pt")
+        c = dict(indexA=torch.stack([ra, ca]), valueA=va, indexB=torch.stack([rb, cb]), valueB=vb,
+                 M=M, K=Kd, N=N, indexC=ic, valueC=vc)
+        cases[name] = sample_spspmm_rows(c, spspmm_keep_rows(c))
+    torch.save({"meta": dict(meta, rows="a quarter of the rows of A (and C)"), "cases": cases}, GOLD / "spspmm2.pt")
+
+
+# ---- row samples: every fixture file stays under 1 MB ---------------------------------------------------------
+def keep_rows(M, must, n, seed):
+    """`must` plus a seeded sample of the other rows, n rows in all, ascending."""
+    must = torch.tensor(sorted(set(must)), dtype=torch.long)
+    rest = torch.ones(M, dtype=torch.bool)
+    rest[must] = False
+    rest = rest.nonzero().flatten()
+    g = torch.Generator().manual_seed(seed)
+    extra = rest[torch.randperm(rest.numel(), generator=g)[:max(n - must.numel(), 0)]]
+    return torch.cat([must, extra]).sort().values
+
+
+def _csr_rows(rowptr, rows):
+    """Entry positions of `rows` (in order) and the rowptr of the CSR made of those rows."""
+    deg = rowptr[rows + 1] - rowptr[rows]
+    new_ptr = torch.zeros(rows.numel() + 1, dtype=torch.long)
+    new_ptr[1:] = torch.cumsum(deg, 0)
+    pos = torch.cat([torch.arange(int(rowptr[r]), int(rowptr[r + 1])) for r in rows.tolist()] +
+                    [torch.empty(0, dtype=torch.long)])
+    return pos, new_ptr
+
+
+def sample_spmm_rows(c, rows):
+    """An spmm_medium case restricted to `rows` of the sparse matrix. Every output row depends on its own entries and
+    `mat` only, so the reference's outputs of those rows are exactly the outputs for the smaller matrix; arg_out
+    positions are renumbered to the smaller entry list (the empty-row sentinel E becomes the new E)."""
+    pos, rowptr = _csr_rows(c["rowptr"], rows)
+    E, E2 = c["col"].numel(), pos.numel()
+    shift = (rowptr[:-1] - c["rowptr"][rows]).view(-1, *([1] * (c["mat"].dim() - 1)))
+    out = dict(rowptr=rowptr, row=torch.repeat_interleave(torch.arange(rows.numel()), rowptr.diff()),
+               col=c["col"][pos], value=c["value"][pos], mat=c["mat"])
+    for k, t in c.items():
+        if k in out:
+            continue
+        t = t[rows]
+        if k.startswith("arg"):
+            t = torch.where(t == E, torch.full_like(t, E2), t + shift)
+        out[k] = t
+    return out
+
+
+def spspmm_keep_rows(c):
+    """Row 0 (empty), the rows with the fewest / most A entries and products, and a seeded sample: M / 4 rows."""
+    (ra, ca), (rb, _) = c["indexA"], c["indexB"]
+    M = c["M"]
+    deg_a = torch.bincount(ra, minlength=M)
+    prods = torch.zeros(M, dtype=torch.long).index_add_(0, ra, torch.bincount(rb, minlength=c["K"])[ca])
+    big = torch.iinfo(torch.long).max
+    must = [0]
+    for m in (deg_a, prods):
+        must += [int(m.argmax()), int(torch.where(m > 0, m, big).argmin())]
+    return keep_rows(M, must, M // 4, seed=84)
+
+
+def sample_spspmm_rows(c, rows):
+    """A SpSpMM case restricted to `rows` of A, renumbered 0..len(rows)-1: row i of C = row i of A times B, so the
+    reference's C restricted to the same rows is the product of the smaller A with B."""
+    new = torch.full((c["M"],), -1, dtype=torch.long)
+    new[rows] = torch.arange(rows.numel())
+    ka, kc = new[c["indexA"][0]] >= 0, new[c["indexC"][0]] >= 0
+    ia, ic = c["indexA"][:, ka].clone(), c["indexC"][:, kc].clone()
+    ia[0], ic[0] = new[ia[0]], new[ic[0]]
+    return dict(c, indexA=ia, valueA=c["valueA"][ka], M=rows.numel(), indexC=ic, valueC=c["valueC"][kc])
 
 
 def gen_grads(ts, meta):
@@ -390,6 +463,30 @@ def gen_grads(ts, meta):
     print("grads.pt", (GOLD / "grads.pt").stat().st_size)
 
 
+def gen_reference_ops(meta):
+    """The reference's compiled CPU operators (ind2ptr / ptr2ind, spmm_sum / mean / min / max over a batched dense
+    operand) for five dtypes, registered as torch.ops.torch_sparse.* by import_reference() or build_ref.load()."""
+    g = torch.Generator().manual_seed(0)
+    M, N, K = 160, 96, 4
+    deg = torch.randint(0, 12, (M,), generator=g)
+    row = torch.repeat_interleave(torch.arange(M), deg)
+    col = torch.randint(N, (row.numel(),), generator=g)
+    rowptr = torch.ops.torch_sparse.ind2ptr(row, M)
+    out = {"meta": meta, "in": dict(row=row, col=col, M=M), "rowptr": rowptr,
+           "row_back": torch.ops.torch_sparse.ptr2ind(rowptr, row.numel()), "cases": {}}
+    for dt in (torch.float32, torch.float64, torch.bfloat16, torch.float16, torch.int64):
+        if dt.is_floating_point:
+            v = torch.randn(col.numel(), generator=g).to(dt); x = torch.randn(2, N, K, generator=g).to(dt)
+        else:
+            v = torch.randint(-5, 6, (col.numel(),), generator=g); x = torch.randint(-5, 6, (2, N, K), generator=g)
+        c = dict(value=v, mat=x, sum=torch.ops.torch_sparse.spmm_sum(None, rowptr, col, v, None, None, x),
+                 mean=torch.ops.torch_sparse.spmm_mean(None, rowptr, col, v, None, None, None, x))
+        c["min"], c["argmin"] = torch.ops.torch_sparse.spmm_min(rowptr, col, v, x)
+        c["max"], c["argmax"] = torch.ops.torch_sparse.spmm_max(rowptr, col, v, x)
+        out["cases"][str(dt).split(".")[-1]] = c
+    torch.save(out, GOLD / "reference_ops.pt")
+
+
 if __name__ == "__main__":
     _meta = {"reference": "rusty1s/pytorch_sparse 0.6.18 @ 91feaa5e", "torch": torch.__version__}
     if len(sys.argv) > 1 and sys.argv[1] == "spspmm2":
@@ -398,5 +495,10 @@ if __name__ == "__main__":
         gen_next_rows2(import_reference(), {"reference": "rusty1s/pytorch_sparse 0.6.18 @ 91feaa5e", "torch": torch.__version__})
     elif len(sys.argv) > 1 and sys.argv[1] == "grads":
         gen_grads(import_reference(), _meta)
+    elif len(sys.argv) > 1 and sys.argv[1] == "reference_ops":   # needs only the operators build_ref.build() makes
+        from oracle import build_ref
+        build_ref.build()
+        build_ref.load()
+        gen_reference_ops(_meta)
     else:
         main()
